@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload decode|prefill|serve|serve8k] [--no-extra] [--no-cpu-baseline]
+                    [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; SURVEY.md section 8d):
 
@@ -34,6 +35,10 @@ Numbers on the JSON line (decode):
             launches (read from the committed capture named in `traffic_source`, null if there is none)
   cpu_baseline  the reference's CPU path (oracle.model: dense bf16 weights, readable operators) on the
             host cores, bounded sample
+
+--dump-outputs DIR (decode) writes what the last timed step handed its caller, rank 0: DIR/logits.npy
+(float32 [1, vocab]) and DIR/next_tokens.npy (the greedy token, float64 [1]).  Weights and prompt are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -150,6 +155,16 @@ def cuda_time_ms(fn, stream=None) -> float:
     return start.elapsed_time(end)
 
 
+def dump_outputs(out_dir: str, **arrays: torch.Tensor) -> None:
+    """Each float32 / float64 tensor as ``out_dir/<name>.npy``."""
+    import numpy as np
+
+    path = Path(out_dir)
+    path.mkdir(parents=True, exist_ok=True)
+    for name, tensor in arrays.items():
+        np.save(path / f"{name}.npy", tensor.cpu().numpy())
+
+
 def base_line(args, world: int, workload: str) -> dict:
     return {
         "metric": METRICS[workload], "value": None, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
@@ -223,6 +238,8 @@ def run_decode(args) -> None:
     barrier(device)
     ms = max_over_ranks(start.elapsed_time(end), device)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the e2e calls below replay the same engine and overwrite its buffers
+        dump_outputs(args.dump_outputs, logits=engine.logits[:1].float(), next_tokens=out_tokens[-1].double())
     # graph replays do not pass through the C ABI; the launches recorded when the step was captured
     # are what each replay executes (plus whatever went through the ABI directly in the region)
     gpu_launches = engine.kernels_per_step * (engine.graph_replays - replays0) + (ext.launch_count() - launches0)
@@ -849,9 +866,14 @@ def main() -> None:
     ap.add_argument("--slots", type=int, default=64, help="serve/serve8k: decode slots per GPU")
     ap.add_argument("--prefill-step", type=int, default=0)
     ap.add_argument("--prompt-len", type=int, default=0, help="prefill: prompt tokens (default 4096)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="decode: write the last timed step's logits and token as DIR/<name>.npy")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"decode": 128, "prefill": 8}.get(args.workload, 0)
+    if args.workload in ("decode", "prefill") and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "decode"):
+        ap.error("--dump-outputs is implemented for --impl ours --workload decode")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "decode":

@@ -2,6 +2,8 @@
 reproduce the operator-by-operator path (same rounding points), and the
 device-resident greedy loop must emit the tokens of the host-driven loop."""
 
+import gc
+
 import pytest
 import torch
 
@@ -307,6 +309,35 @@ def test_device_resident_greedy_loop_equals_host_driven_loop(dev, tiny_gpu):
     dev_tokens, dev_state = run(True)
     assert dev_tokens == host_tokens
     assert dev_state == host_state == ([0, 1, 2, 3], [8, 8, 8, 7], 31)
+
+
+def test_no_garbage_collection_starts_while_an_engine_captures(dev, tiny_gpu):
+    """An engine and its model reference each other, so a dropped model's CUDA graphs are freed by the cyclic
+    collector, and destroying a graph while a stream captures invalidates that capture.  With a collection due at
+    almost every allocation, none may start inside the decode or the prefill engine's capture."""
+    capturing = []
+
+    def watch(phase, info):
+        if phase == "start":
+            capturing.append(torch.cuda.is_current_stream_capturing())
+
+    model = Qwen3ModelWeek3(tiny_gpu, page_size=64)  # 64-token pages: prefill chunks run on the prefill engine
+    cache, tok = prefill(model, dev, [9, 2, 4, 6, 8])
+    gc.collect()  # engines dropped by earlier tests go now, outside any capture
+    threshold = gc.get_threshold()
+    gc.callbacks.append(watch)
+    gc.set_threshold(1)
+    try:
+        model(torch.tensor([[tok]], dtype=torch.int32, device=dev), 5, cache, logits_to_keep=1)  # decode engine capture
+        second = model.create_kv_cache()
+        model(torch.tensor([[1, 5, 7]], dtype=torch.int32, device=dev), 0, second, logits_to_keep=1)  # prefill engine capture
+    finally:
+        gc.set_threshold(*threshold)
+        gc.callbacks.remove(watch)
+    for c in (*cache, *second):
+        c.release()
+    assert model._decode_engines and model._prefill_engines
+    assert capturing and not any(capturing)
 
 
 def test_public_model_call_uses_the_graph_and_matches_operator_path(dev, tiny_gpu):

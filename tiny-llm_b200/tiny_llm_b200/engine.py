@@ -25,6 +25,8 @@ front and the engine re-captures if a slab pointer changes.
 
 from __future__ import annotations
 
+import contextlib
+import gc
 import os
 
 from types import SimpleNamespace
@@ -36,6 +38,20 @@ from extensions_b200 import tiny_llm_ext_b200 as ext
 
 from .kv_cache import BatchingKvCache
 from .paged_kv_cache import TinyKvPagedCache
+
+
+@contextlib.contextmanager
+def _gc_paused():
+    """No cyclic garbage collection during a graph capture.  An engine and its model reference each other, so a
+    dropped model is freed by the collector; destroying its CUDA graphs while a stream captures is a CUDA call
+    that capture forbids, and it invalidates the capture in progress."""
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        yield
+    finally:
+        if enabled:
+            gc.enable()
 
 
 def _concat_weights(parts):
@@ -303,7 +319,7 @@ class DecodeEngine:
         self.captures += 1
         self._slab_ptrs = self._slabs()
         forward = self._forward_fused if self.fused else self._forward_unfused
-        with torch.cuda.stream(self._stream):
+        with torch.cuda.stream(self._stream), _gc_paused():
             self._stream.wait_stream(torch.cuda.current_stream(self.device))
             # The warm-up passes really run: with the previous step's metadata still on the device they
             # would append a stale token's K/V through a stale block table - possibly into a page that
@@ -672,7 +688,7 @@ class PrefillEngine:
     def _capture(self) -> None:
         self.captures += 1
         self._slab_ptrs = self._slabs()
-        with torch.cuda.stream(self._stream):
+        with torch.cuda.stream(self._stream), _gc_paused():
             self._stream.wait_stream(torch.cuda.current_stream(self.device))
             # warm-up passes run for real: all rows padding (context 0 -> no append), no visible keys
             self.meta_dev[2 * self.L:3 * self.L + 1].zero_()
